@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5                       # this framework, cfg2 per GPU
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference --steps K --warmup W               # the oracle port on the host CPU cores
+    python bench.py --steps K --warmup W --dump-outputs DIR              # also DIR/sample.npy, DIR/pred_xstart.npy of the last timed step
 
 A "step" is one ddim_sample_with_grad iteration (UNet fwd -> cutouts -> CLIP ViT fwd/bwd -> losses -> UNet dgrad ->
 DDIM update) of BASELINE.json configs[1]: 256x256, ddim250, 1 image per GPU, 16 cutouts, ViT-B/32, synthetic noise and
@@ -46,6 +47,7 @@ WORKLOADS = {
 CFG = WORKLOADS["cfg2"]
 FLOP_PER_IMAGE_STEP = 4.775e12  # SURVEY.md 8d: UNet 2.240+2.252, CLIP 0.141+0.143 TFLOP (fwd + dgrad)
 DOMINANT = dict(M=65536, N=256, K=2304)  # 256^2 x 256ch conv3x3: 31 % of the UNet FLOPs (SURVEY App. C)
+DUMP_BYTES = 64 << 20  # --dump-outputs: the .npy files together stay below this
 
 
 def peaks():
@@ -59,6 +61,20 @@ def peaks():
         except (OSError, ValueError, KeyError, TypeError):  # unreadable / other schema: say "fallback" rather than abort the bench line
             pass
     return fb
+
+
+def dump_outputs(path, arrays):
+    """One float32 DIR/<name>.npy per array.  Above DUMP_BYTES in all, each array is cut to the same fixed, seeded sample of its
+    flattened elements on every run, so that two builds' dumps stay comparable element for element."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(a.numel() * 4 for a in arrays.values())
+    budget = DUMP_BYTES - 1024 * len(arrays)  # room for the .npy headers
+    for name, a in arrays.items():
+        if total > budget:
+            keep = a.numel() * budget // total
+            a = a.flatten()[th.randperm(a.numel(), generator=th.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(path, f"{name}.npy"), a.numpy())
 
 
 class ClockSampler:
@@ -230,6 +246,7 @@ def run_ours(args):
     B = eng.B
     T = diff.num_timesteps
     y0 = th.zeros(eng.global_batch, dtype=th.long)
+    last = {}
 
     def step_resident(i, img):
         # x_t is fresh synthetic noise every step: with random (non-denoising) weights a chained trajectory diverges within a
@@ -238,6 +255,7 @@ def run_ours(args):
         y = eng.draw_classes()
         out = eng.fused_step(diff, MODE, i, img, y, cond, 0.0)
         cond.current_timestep = max(cond.current_timestep - 1, 0)
+        last.update(out)
         return out["sample"]
 
     # ---------------- device-resident loop (value)
@@ -270,6 +288,11 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     ms_total = float(ms.item())
     finite = bool(th.isfinite(img).all()) and tuple(gathered.shape) == (eng.global_batch, 3, eng.H, eng.W)
+    if args.dump_outputs:
+        # what the last timed step returned, every rank's rows in rank order; .cpu() before the next gather reuses its buffer
+        outs = {k: eng.gather_final(v).cpu() for k, v in sorted(last.items())}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
 
     # ---------------- end-to-end loop: host buffers, H2D of x_t and D2H of the sample inside every step
     host_x = th.empty(B, 3, eng.H, eng.W, pin_memory=True)
@@ -489,31 +512,18 @@ def cpu_baseline(sample_steps=3):
 def run_reference(args):
     """The reference's own algorithm on the host cores (fp32 oracle port: guided_diffusion / clip / lpips are not installable
     offline, DESIGN.md section 5).  Same metric / unit / config strings as our arm; --warmup W untimed steps, --steps K timed ones.
-    One cfg2 step is 5-6 s on the B200 host: W + K steps fit a few minutes; on a slower host the run is cut to a time budget and
-    says so (`steps` / `warmup` then report what actually ran)."""
+    One cfg2 step takes 5-6 s on a B200 host's CPU cores."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     unet, diff, cond = oracle_cpu_setup()
-    budget_s = float(os.environ.get("CGD_REF_BUDGET_S", "240"))
-    t_last, x = oracle_cpu_steps(unet, diff, cond, 1)  # cold step (allocator, thread pool): always run, the first warm-up step
-    warm_done, n_timed = 1, args.steps
-    if args.warmup >= 2:
-        t_last, x = oracle_cpu_steps(unet, diff, cond, 1, x)  # a warm step sizes the rest of the run
-        warm_done = 2
-    per = t_last[0]
-    more_warm = max(args.warmup - warm_done, 0)
-    if per * (more_warm + n_timed) > budget_s:  # slow host: drop the remaining warm-up first, then cut the timed sample
-        more_warm = 0
-        n_timed = int(max(1, min(args.steps, budget_s // per)))
-    if more_warm:
-        _, x = oracle_cpu_steps(unet, diff, cond, more_warm, x)
-        warm_done += more_warm
+    _, x = oracle_cpu_steps(unet, diff, cond, args.warmup)  # the first one is the cold step (allocator, thread pool)
+    n_timed = args.steps
     times, _ = oracle_cpu_steps(unet, diff, cond, n_timed, x)
     total = float(sum(times))
     value = n_timed / total
     line = {"impl": "reference", "metric": "diffusion-steps/sec", "value": value,
             "unit": f"image-steps/s (1 step of one {CFG['image_size']}x{CFG['image_size']} image, {CFG['cutn']} cutouts)",
-            "n_gpus": args.gpus, "steps": n_timed, "requested_steps": args.steps, "warmup": warm_done,
+            "n_gpus": args.gpus, "steps": n_timed, "warmup": args.warmup,
             "ms_per_step": total / n_timed * 1e3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "fp32", "data": "synthetic (seeded random weights)",
             "config": {"workload": CFG["name"] + ", class-cond UNet, seeded random weights", "global_batch": 1,
@@ -521,7 +531,7 @@ def run_reference(args):
                        "note": "the reference's own algorithm as the fp32 oracle port on the host CPU; guided_diffusion / clip are not "
                                "installable offline"},
             "cpu_baseline": {"value": value, "unit": "image-steps/s", "cores": pick_cpu_threads(), "host_cpus": os.cpu_count(), "kind": "port",
-                             "sample": f"{n_timed} full cfg2 steps after {warm_done} untimed (time budget {budget_s:.0f} s; {args.steps} requested)"},
+                             "sample": f"{n_timed} full cfg2 steps after {args.warmup} untimed"},
             "e2e": {"value": value, "unit": "image-steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line))
@@ -537,7 +547,13 @@ def main():
     ap.add_argument("--no-torch-baseline", action="store_true", help="skip the PyTorch-CUDA (cuDNN/cuBLAS eager autograd) oracle-port arm")
     ap.add_argument("--torch-baseline", action="store_true", help="(default now; kept for old command lines)")
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS), help="per-GPU shard of a BASELINE.json configuration (default: the metric's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's sample and pred_xstart "
+                                                          "(float32, the whole batch) to DIR/<name>.npy; same arguments, same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
     global CFG
     CFG = WORKLOADS[args.workload]
     args.warmup = max(args.warmup, 3)

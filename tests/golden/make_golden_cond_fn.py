@@ -8,7 +8,7 @@ deterministic "CLIP" (`StubClip`) and a deterministic `pred_xstart = f(x)` in pl
 closure itself does: the x_in blend with the float64 `fac`, normalisation, the view / broadcast of the spherical loss, the weighting and
 reduction of every term, the saturation term, the sign, the whole-batch RMS clamp, the reduce_clip / progressive_cutout schedules.
 
-    python tests/golden/make_golden_cond_fn.py        # writes tests/golden/cond_fn_golden.npz (committed); needs /root/reference
+    CGD_REFERENCE=<reference checkout> python tests/golden/make_golden_cond_fn.py      # writes tests/golden/cond_fn_golden.npz (committed)
 """
 import ast
 import json
@@ -21,20 +21,21 @@ import torch as th
 import torch.nn.functional as F
 import torchvision.transforms as tvt
 
-sys.path.insert(0, "/root/reference")
+REF = os.environ["CGD_REFERENCE"]  # a checkout of the reference repository
+sys.path.insert(0, REF)
 from cgd import losses  # noqa: E402  (the reference's own module)
 from cgd.modules import MakeCutouts  # noqa: E402  (the reference's own module)
 
 
 def reference_cond_fn_code():
-    tree = ast.parse(open("/root/reference/cgd/cgd.py").read())
+    tree = ast.parse(open(os.path.join(REF, "cgd", "cgd.py")).read())
     outer = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "clip_guided_diffusion")
     fn = next(n for n in ast.walk(outer) if isinstance(n, ast.FunctionDef) and n.name == "cond_fn")
     return compile(ast.Module([fn], []), "cgd/cgd.py", "exec")
 
 
 def reference_clip_normalize():
-    tree = ast.parse(open("/root/reference/cgd/clip_util.py").read())
+    tree = ast.parse(open(os.path.join(REF, "cgd", "clip_util.py")).read())
     node = next(n for n in tree.body if isinstance(n, ast.Assign) and getattr(n.targets[0], "id", "") == "CLIP_NORMALIZE")
     return eval(compile(ast.Expression(node.value), "cgd/clip_util.py", "eval"), {"tvt": tvt})
 
